@@ -40,6 +40,32 @@ C3_NAME = ("C3: 1M pods = 1000 apps x 1000 replicas, topologySpread(zone, maxSke
 C2_NAME = "C2: 100k pods with zone/arch nodeSelector + tolerations, first 500 AWS-KWOK instance types, 1 tainted NodePool"
 C5_NAME = ("C5: 10M pods, 8 NodePools (pods pinned by nodeSelector + toleration), half C2 mix / half C3 mix (apps of "
            "1000 replicas, never across pools), first 1000 AWS-KWOK instance types; NodePool p on rank p mod N")
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much in all
+
+
+def exact_f64(v):
+    """float64 copy of an integer result array that keeps every value exact: a 64-bit word becomes its (high, low)
+    32-bit halves along a new last axis."""
+    a = np.asarray(v)
+    if a.dtype.itemsize == 8 and a.dtype.kind in "iu":
+        a = np.stack([a >> 32, a & 0xFFFFFFFF], axis=-1)
+    return a.astype(np.float64)
+
+
+def dump_outputs(out_dir, res, keys, limit=DUMP_BYTES):
+    """Writes res[k] as out_dir/<k>.npy (float64, see exact_f64) for every k in keys.  When the arrays exceed `limit`
+    bytes, every array keeps the same fraction of its rows, sorted, drawn with the array's length as the seed: arrays of
+    one length (all the per-pod ones) keep the same rows, and two runs of the same workload keep the same rows."""
+    arrays = {k: exact_f64(res[k]) for k in keys}
+    budget = limit - 4096 * len(arrays)  # room for the .npy headers
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        if total > budget and a.ndim > 0 and len(a) > 1:
+            n = len(a)
+            rows = np.random.default_rng(n).choice(n, max(1, n * budget // total), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def algorithmic_bytes(res, n_pods, n_its, n_groups=0, domains=4):
@@ -469,16 +495,23 @@ def main():
     ap.add_argument("--no-c5", action="store_true")
     ap.add_argument("--consol-nodes", type=int, default=10_000)
     ap.add_argument("--consol-pods", type=int, default=200_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline's result of its last timed step as DIR/<name>.npy (float64, one file per "
+                         "result array of the C ABI), so that two builds can be compared output for output")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (world > 1 or args.impl != "karpsolve"):
+        ap.error("--dump-outputs writes the one-GPU headline (C3) of --impl karpsolve")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
     import torch
     import torch.distributed as dist
-    from karpenter_b200 import _native, workloads
+    from karpenter_b200 import _abi, _native, workloads
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
@@ -501,6 +534,8 @@ def main():
         n_pods = args.apps * C3_REPLICAS
         m = time_provisioning(h, enc.problem, n_pods, args.steps, args.warmup, torch, flush, barrier, sampler)
         res, st = m["res"], m["stats"]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, res, _abi.PARITY_KEYS)
         name = C3_NAME if args.apps == C3_APPS else C3_NAME.replace("1M pods = 1000 apps", f"{n_pods} pods = {args.apps} apps")
         line = {
             "metric": "pods scheduled/sec", "value": n_pods / (m["ms"] / 1000), "unit": "pods/s", "n_gpus": 1,
